@@ -249,6 +249,8 @@ def reference_arm(args):
     if ref is not None:
         line["relmse"] = {"reference_algorithm": relmse(vals[-1]["image"], ref), "spp": budget, "against": f"scenes/ref/{args.scene}_{w}x{h}_ref.npy"}
     emit_line(line)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"film": vals[-1]["image"]})
 
 
 # ------------------------------------------------------------------------------------------- GPU arm
@@ -294,12 +296,14 @@ def gpu_arm(args):
     sampler.region(True)
     t0 = time.perf_counter()
     stats = []
+    film_ptr = None
     for _ in range(args.steps):
-        _, st = g.render_device()
+        film_ptr, st = g.render_device()
         stats.append(st)
     barrier()
     wall = time.perf_counter() - t0
     sampler.region(False)
+    film = device_film(film_ptr, args.height, args.width) if args.dump_outputs and rank == 0 else None     # before the e2e steps reuse the film buffer
     dev_ms = sum(s["render_device_ms"] for s in stats)          # CUDA events on the library's launching stream
     verts = sum(s["total_vertices"] for s in stats); paths = sum(s["total_paths"] for s in stats)
     launches = sum(s["kernel_launches"] for s in stats)
@@ -405,8 +409,41 @@ def gpu_arm(args):
             print({k: (round(v, 4) if isinstance(v, float) else v) for k, v in it.items() if k in ("iteration", "passes", "seconds", "reset_seconds", "build_seconds", "variance", "s_tree_leaves", "vertices", "nodes_avg", "depth_avg", "s_tree_depth_avg")}, file=sys.stderr)
         print({"render_device_ms": stats[-1]["render_device_ms"], "render_seconds": stats[-1]["render_seconds"], "kernel_ms": stats[-1]["kernel_ms"]}, file=sys.stderr)
     emit_line(line)
+    if film is not None:
+        dump_outputs(args.dump_outputs, {"film": film})
     if dist is not None:
         dist.destroy_process_group()
+
+
+def device_film(ptr, h, w):
+    """Host copy of the H x W x 3 float32 film that ppg_render_device left in HBM."""
+    import torch
+
+    class _Film:
+        __cuda_array_interface__ = {"shape": (h, w, 3), "typestr": "<f4", "data": (ptr, False), "version": 3}
+    torch.cuda.synchronize()
+    return torch.as_tensor(_Film(), device="cuda").cpu().numpy().copy()
+
+
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: what the timed path returned in its last step, one DIR/<name>.npy per array (float32 / float64), so that two
+    builds run with the same arguments (same scene, same seed) can be compared output for output.  A film larger than 64 MB is
+    stored as a fixed, seeded sample of its pixels: DIR/<name>_sample.npy (N x 3) and the flat pixel indices DIR/<name>_sample_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        if a.nbytes <= DUMP_LIMIT:
+            np.save(os.path.join(out_dir, name + ".npy"), a)
+            continue
+        px = a.reshape(-1, a.shape[-1])
+        n = DUMP_LIMIT // 2 // px[0].nbytes
+        idx = np.sort(np.random.default_rng(0).choice(len(px), n, replace=False))
+        np.save(os.path.join(out_dir, name + "_sample.npy"), px[idx])
+        np.save(os.path.join(out_dir, name + "_sample_index.npy"), idx.astype(np.float64))
 
 
 _REAL_STDOUT = None
@@ -444,7 +481,11 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=150.0, help="reference arm: stop repeating once this much time has been spent")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--verbose", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the film of the last timed step (H x W x 3 float32) as DIR/film.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     quiet_stdout()
     _, W, H, spp, _ = SCENES[args.scene]
     args.width = args.size or W

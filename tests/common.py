@@ -5,6 +5,22 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
+def reference_dir():
+    """A checkout of the original project (Tom94/practical-path-guiding), for the few checks that need its large scene assets (SPACESHIP 52 MB,
+    KITCHEN 140 MB, the Stanford bunny): PPG_REFERENCE_DIR, else the checkout the package reads Mitsuba's data files from
+    (ppg_b200.rtrans: <checkout>/mitsuba/data/microfacet).  Those checks skip where neither exists."""
+    if os.environ.get("PPG_REFERENCE_DIR"):
+        return os.environ["PPG_REFERENCE_DIR"]
+    from ppg_b200 import rtrans
+    return os.path.dirname(os.path.dirname(os.path.dirname(rtrans._DATA_DIR)))
+
+
+def reference_file(*parts):
+    """Path of a file of the original project's checkout, or None where there is none."""
+    p = os.path.join(reference_dir(), *parts)
+    return p if os.path.exists(p) else None
+
+
 def assert_render_parity(img, ref, st, ost, sc=None, props=None, pixels=0.90, mean=0.01, counts=2e-4, leaves=1):
     """Parity of a TRAINED render of the CUDA path (img, st) with the oracle's (ref, ost) on the same seeded inputs.
 
@@ -56,6 +72,23 @@ def load_fixture_scene(name, size=None):  # size None or 0: the XML film size
 def relmse(img, ref):
     img = np.asarray(img, np.float64); ref = np.asarray(ref, np.float64)
     return float(np.mean((img - ref) ** 2 / (ref ** 2 + 1e-3)))
+
+
+def load_rough_transmittance(dist):
+    """Mitsuba's data/microfacet/<dist>.dat as ppg_b200.rtrans.load_table returns it, rebuilt from tests/golden/rough_transmittance_<dist>.npz
+    (tools/make_golden.py): the nodes the rough plastics of the tests interpolate; every other node is NaN."""
+    z = np.load(os.path.join(ROOT, "tests", "golden", f"rough_transmittance_{dist}.npz"))
+    n_eta, n_alpha, n_theta = (int(v) for v in z["shape"])
+    trans = np.full((2 * n_eta, n_alpha, n_theta), np.nan, np.float32); diff = np.full((2 * n_eta, n_alpha), np.nan, np.float32)
+    trans[z["index"][:, 0], z["index"][:, 1]] = z["trans"]; diff[z["index"][:, 0], z["index"][:, 1]] = z["diff"]
+    r = z["ranges"]
+    return dict(trans=trans, diff=diff, n_eta=n_eta, n_alpha=n_alpha, n_theta=n_theta, eta_min=r[0], eta_max=r[1], alpha_min=r[2], alpha_max=r[3])
+
+
+def load_sky_tables():
+    """datasetRGB1-3 / datasetRGBRad1-3 of Mitsuba's skymodeldata.h as ppg_b200.sunsky._sky_tables returns them (tests/golden/sky_model_rgb.npz)."""
+    z = np.load(os.path.join(ROOT, "tests", "golden", "sky_model_rgb.npz"))
+    return {k: z[k] for k in z.files}
 
 
 def gpu_available():

@@ -116,8 +116,6 @@ def test_device_triangle_test_and_transmittance_sources_equal_the_reference(dev)
     dev.dev_tri_intersect(n, k.ctypes.data_as(C.POINTER(C.c_int)), c9.ctypes.data_as(f32p), arrs[3].ctypes.data_as(f32p), arrs[4].ctypes.data_as(f32p), mint.ctypes.data_as(f32p),
                           maxt.ctypes.data_as(f32p), hit2.ctypes.data_as(C.POINTER(C.c_ubyte)), tuv2.ctypes.data_as(f32p))
     assert 0.1 < hit.mean() < 0.5 and np.array_equal(hit, hit2) and np.array_equal(tuv[hit == 1], tuv2[hit == 1])
-    if not __import__("os").path.exists("/root/reference/mitsuba/data/microfacet/ggx.dat"):
-        return                                                              # (the table comes from the reference's data files)
     from ppg_b200 import rtrans
     lut, _ = rtrans.reduce_for_material("beckmann", 1.49, 0.1); lut = np.ascontiguousarray(lut, np.float32)
     cs = np.concatenate([rng.uniform(-0.2, 1, 100000), [0.0, 1.0]]).astype(np.float32)
@@ -131,12 +129,10 @@ def test_device_triangle_test_and_transmittance_sources_equal_the_reference(dev)
 
 def _material(name):
     """One BSDF configuration of the hot path (DESIGN.md 1.1) with the wrappers that change its arithmetic: (ppg_bsdf, tables).  Built inside the test: the
-    rough-plastic tables are reduced from the reference's data files, which exist only where /root/reference does."""
+    rough-plastic tables are reduced from the nodes of Mitsuba's data files stored under tests/golden."""
     from ppg_b200 import scene as S
     mk = lambda **kw: O.make_bsdf(**kw)
     if name in ROUGHPLASTICS:
-        if not os.path.exists("/root/reference/mitsuba/data/microfacet/ggx.dat"):
-            pytest.skip("the rough-transmittance tables of the reference are not present")
         tables = []
         row = S.make_roughplastic(*ROUGHPLASTICS[name], tables)
         return O.bsdf_from_row(row), np.ascontiguousarray(tables, np.float32)

@@ -8,7 +8,7 @@ import sys
 import numpy as np
 import pytest
 
-from common import ROOT, gpu_available, load_cbox
+from common import ROOT, gpu_available, load_cbox, reference_file
 from ppg_b200 import capi, integrator as I
 
 
@@ -97,21 +97,21 @@ def test_cbox_rgb_values_match_mitsubas_spectrum_conversion():
     assert len(sc.indices) == 36
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/scenes/cbox/cbox.xml"), reason="reference tree not present")
 def test_fixture_is_what_the_loader_produces_from_the_reference_xml():
+    """scenes/cbox.npz is the loader's output for the original project's scenes/cbox/cbox.xml (stored with its meshes under tests/golden/cbox)."""
     from ppg_b200.scene import load_mitsuba_xml
-    a = load_mitsuba_xml("/root/reference/scenes/cbox/cbox.xml"); b = load_cbox()
+    a = load_mitsuba_xml(os.path.join(ROOT, "tests", "golden", "cbox", "cbox.xml")); b = load_cbox()
     for k in ("positions", "normals", "indices", "triangle_shape", "shapes", "bsdfs", "area_radiance", "cam_to_world", "aabb_min", "aabb_max"):
         assert np.array_equal(getattr(a, k), getattr(b, k)), k
     assert a.integrator == b.integrator and a.x_fov_deg == b.x_fov_deg
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/scenes/spaceship/spaceship-improved.xml"), reason="reference tree not present")
+@pytest.mark.skipif(reference_file("scenes", "spaceship", "spaceship-improved.xml") is None, reason="needs the original project's SPACESHIP assets (tests/common.py: reference_dir)")
 def test_spaceship_fixture_is_what_the_loader_produces_from_the_reference_xml():
     """spaceship-improved.xml exercises the whole loader: matrix transforms, OBJ meshes with faceNormals, rectangles, a sphere with
     flipNormals, twosided wrappers, roughconductor / roughplastic (reduced transmittance tables) / roughdielectric, named and referenced BSDFs."""
     from ppg_b200.scene import load_mitsuba_xml, SceneDesc
-    a = load_mitsuba_xml("/root/reference/scenes/spaceship/spaceship-improved.xml")
+    a = load_mitsuba_xml(reference_file("scenes", "spaceship", "spaceship-improved.xml"))
     b = SceneDesc.load(os.path.join(ROOT, "scenes", "spaceship-improved.npz"))
     for k in ("positions", "normals", "indices", "triangle_shape", "shapes", "bsdfs", "bsdf_tables", "spheres", "area_radiance", "cam_to_world", "aabb_min", "aabb_max"):
         assert np.array_equal(getattr(a, k), getattr(b, k)), k
@@ -121,7 +121,6 @@ def test_spaceship_fixture_is_what_the_loader_produces_from_the_reference_xml():
     assert a.integrator["bsdfSamplingFractionLoss"] == "kl" and a.integrator["sppPerPass"] == "1"
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/mitsuba/data/microfacet/beckmann.dat"), reason="reference tree not present")
 def test_rough_transmittance_reduction_has_the_physical_limits():
     """rtrans.py (= RoughTransmittance::setEta/setAlpha/evalDiffuse): at low roughness the table tends to 1 - Fresnel; the diffuse
     internal reflectance matches fresnelDiffuseReflectance(1/eta) (both integrate the same quantity for a smooth interface)."""
@@ -160,11 +159,11 @@ def test_unsupported_scene_content_is_refused_not_substituted(tmp_path):
             load_mitsuba_xml(str(p))
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/scenes/kitchen/kitchen-improved.xml"), reason="reference tree not present")
+@pytest.mark.skipif(reference_file("scenes", "kitchen", "kitchen-improved.xml") is None, reason="needs the original project's KITCHEN assets (tests/common.py: reference_dir)")
 def test_kitchen_fixture_is_what_the_loader_produces_from_the_reference_xml():
     """kitchen-improved.xml (BASELINE config 3): 291 OBJ meshes, 13 bitmap textures, the sunsky emitter, bump maps whose nested BSDF carries the id."""
     from ppg_b200.scene import load_mitsuba_xml, SceneDesc, BSDF_FLAG_BUMPMAP
-    a = load_mitsuba_xml("/root/reference/scenes/kitchen/kitchen-improved.xml")
+    a = load_mitsuba_xml(reference_file("scenes", "kitchen", "kitchen-improved.xml"))
     b = SceneDesc.load(os.path.join(ROOT, "scenes", "kitchen-improved.npz"))
     for k in ("positions", "normals", "uvs", "indices", "triangle_shape", "shapes", "bsdfs", "bsdf_tables", "area_radiance", "cam_to_world", "aabb_min", "aabb_max", "texels"):
         assert np.array_equal(getattr(a, k), getattr(b, k)), k
@@ -414,8 +413,8 @@ def test_loader_reads_ply_meshes(tmp_path):
     (tmp_path / "m.xml").write_text(_scene_xml('<shape type="ply"><string name="filename" value="le.ply"/><boolean name="faceNormals" value="true"/><boolean name="flipNormals" value="true"/><bsdf type="diffuse"/></shape>'))
     sc = S.load_mitsuba_xml(str(tmp_path / "m.xml"))
     assert sc.shapes[1, 1] == 4 and sc.shapes[1, 4] == 0 and sc.indices[2:].tolist() == (np.array([[1, 0, 2], [3, 2, 4], [2, 5, 4], [5, 4, 6]]) + 4).tolist()
-    bunny = "/root/reference/mitsuba/data/tests/bunny.ply"                          # the mesh of the reference's test_kd.cpp
-    if os.path.exists(bunny):
+    bunny = reference_file("mitsuba", "data", "tests", "bunny.ply")                # the mesh of the reference's test_kd.cpp
+    if bunny is not None:
         P, N, uv, I = S._load_ply(bunny, np.eye(4))
         assert P.shape == (35947, 3) and I.shape == (69451, 3) and uv is None and np.allclose(np.linalg.norm(N, axis=1), 1, atol=1e-4)
         ctr = P.mean(0); tri = P[I]; fn = np.cross(tri[:, 1] - tri[:, 0], tri[:, 2] - tri[:, 0])

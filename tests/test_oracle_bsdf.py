@@ -4,6 +4,9 @@ import numpy as np
 import pytest
 
 import oracle_lib as O
+from reference_outputs import reference
+
+HAVE_MFREF = __import__("os").path.exists(O.MFREF_SO)      # the reference's own functions (oracle/_ref), else the rows stored under tests/golden
 
 CASES = {
     "diffuse": dict(type=0, reflectance=(0.6, 0.5, 0.4)),
@@ -19,7 +22,7 @@ CASES = {
 
 
 def _roughplastic(distribution, alpha, nonlinear, diffuse=(0.256, 0.013, 0.08)):
-    """(ppg_bsdf, tables) through the host loader's reduction of the reference's data/microfacet tables (rtrans.py)."""
+    """(ppg_bsdf, tables) through the host loader's reduction of Mitsuba's data/microfacet tables (rtrans.py; the nodes stored under tests/golden)."""
     from ppg_b200.scene import make_roughplastic
     tables = []
     row = make_roughplastic(0, diffuse, (1, 1, 1), 1.5 / 1.000277, alpha, distribution, nonlinear, tables)
@@ -143,15 +146,17 @@ def test_oracle_looks_through_null_surfaces_consistently():
     assert 1.1 * mean["never"] < mean["always"] < 1.6 * mean["never"]
 
 
-@pytest.mark.skipif(not __import__("os").path.exists(O.MFREF_SO), reason="oracle/_ref/libmicrofacet_ref.so not built (needs /root/reference at build time)")
 @pytest.mark.parametrize("type_", [0, 1])          # PPG_MICROFACET_BECKMANN, PPG_MICROFACET_GGX
 @pytest.mark.parametrize("alpha", [0.01, 0.1, 0.2, 0.6])
 def test_restated_microfacet_equals_the_reference_class(type_, alpha):
     """The oracle's microfacet restatement (struct Microfacet of ppg_cpu_tracer.h: D, Smith G1, the Heitz-d'Eon visible-normal sampling with its Newton
     iteration / rational fits, and mts_erf / mts_erfinv) against the reference's OWN class MicrofacetDistribution (src/bsdfs/microfacet.h:45-721) and math::erf /
     erfinv (src/libcore/math.cpp:25-72) compiled verbatim: same inputs, every float must agree bit for bit (both sides are built without FMA contraction and
-    call the same libm).  This is what roughconductor / roughplastic / roughdielectric are built on -- and what the CUDA mf_* functions mirror."""
-    ref, port = O.microfacet("ref"), O.microfacet("port")
+    call the same libm).  This is what roughconductor / roughplastic / roughdielectric are built on -- and what the CUDA mf_* functions mirror.
+    Without oracle/_ref the reference's outputs are the rows stored under tests/golden (tests/reference_outputs.py)."""
+    ref, port = (O.microfacet("ref") if HAVE_MFREF else None), O.microfacet("port")
+    live = lambda f: f if HAVE_MFREF else None
+    key = f"microfacet/{type_}/{alpha}"
     rng = np.random.default_rng(100 * type_ + int(alpha * 100))
     n = 200000
     def dirs(upper):
@@ -162,45 +167,54 @@ def test_restated_microfacet_equals_the_reference_class(type_, alpha):
     m, v, wi = dirs(False), dirs(False), dirs(True)
     # grazing and near-normal incidence, where the sampling code switches branches (theta < 1e-4, cot / tan extremes)
     wi[:1000] = [0, 0, 1]; wi[1000:2000, 2] = 1e-3 * rng.random(1000); wi[1000:2000] /= np.linalg.norm(wi[1000:2000], axis=1, keepdims=True)
-    assert np.array_equal(ref.eval(type_, alpha, m), port.eval(type_, alpha, m))
-    assert np.array_equal(ref.smith_g1(type_, alpha, v, m), port.smith_g1(type_, alpha, v, m))
-    assert np.array_equal(ref.pdf(type_, alpha, wi, np.abs(m)), port.pdf(type_, alpha, wi, np.abs(m)))
+    ma = np.abs(m)
+    i, (e, g, p) = reference(key, live(lambda: [ref.eval(type_, alpha, m), ref.smith_g1(type_, alpha, v, m), ref.pdf(type_, alpha, wi, ma)]), n)
+    assert np.array_equal(e, port.eval(type_, alpha, m[i]))
+    assert np.array_equal(g, port.smith_g1(type_, alpha, v[i], m[i]))
+    assert np.array_equal(p, port.pdf(type_, alpha, wi[i], ma[i]))
     smp = rng.random((n, 2), dtype=np.float32); smp[:50] = [[0.0, 0.0]] * 50; smp[50:100] = [[0.99999994, 0.99999994]] * 50
-    mr, pr = ref.sample(type_, alpha, wi, smp); mp, pp = port.sample(type_, alpha, wi, smp)
+    i, (mr, pr) = reference(key + "/sample", live(lambda: ref.sample(type_, alpha, wi, smp)), n)
+    _, (ok_frac,) = reference(key + "/sample_finite", live(lambda: [np.array([np.isfinite(ref.sample(type_, alpha, wi, smp)[0]).all(axis=1).mean()])]), 1)
+    mp, pp = port.sample(type_, alpha, wi[i], smp[i])
     ok = np.isfinite(mr).all(axis=1)
-    assert ok.mean() > 0.999 and np.array_equal(np.isfinite(mp).all(axis=1), ok)
+    assert ok_frac[0] > 0.999 and np.array_equal(np.isfinite(mp).all(axis=1), ok)
     assert np.array_equal(mr[ok], mp[ok]) and np.array_equal(pr[ok], pp[ok])
     x = np.concatenate([rng.uniform(-0.999999, 0.999999, 100000), [-0.99999994, 0.0, 0.99999994], rng.uniform(-6, 6, 1000)]).astype(np.float32)
-    er, eir = ref.erf(x); ep, eip = port.erf(x)
-    assert np.array_equal(er, ep) and np.array_equal(eir[np.abs(x) < 1], eip[np.abs(x) < 1])
+    i, (er, eir) = reference(key + "/erf", live(lambda: ref.erf(x)), len(x))
+    ep, eip = port.erf(x[i]); inside = np.abs(x[i]) < 1
+    assert np.array_equal(er, ep) and np.array_equal(eir[inside], eip[inside])
 
 
-@pytest.mark.skipif(not __import__("os").path.exists(O.MFREF_SO), reason="oracle/_ref/libmicrofacet_ref.so not built (needs /root/reference at build time)")
 def test_restated_helpers_equal_the_reference_functions():
     """fresnelDielectricExt, the Spectrum overload of fresnelConductorExact, coordinateSystem (src/libcore/util.cpp:592-601, 651-681, 739-761) and
     warp::squareToCosineHemisphere (warp.cpp:43-52, 81-102), compiled verbatim, against the oracle's restatements: bit for bit."""
-    ref, port = O.microfacet("ref"), O.microfacet("port")
+    ref, port = (O.microfacet("ref") if HAVE_MFREF else None), O.microfacet("port")
+    live = lambda f: f if HAVE_MFREF else None
     rng = np.random.default_rng(9)
     c = np.concatenate([rng.uniform(-1, 1, 200000), [0.0, 1.0, -1.0, 1e-6, -1e-6]]).astype(np.float32)
     for eta in (1.0, 1.5046 / 1.000277, 1 / 1.5, 1.33, 2.4):
-        fr, tr = ref.fresnel_dielectric_ext(c, eta); fp, tp = port.fresnel_dielectric_ext(c, eta)
+        i, (fr, tr) = reference(f"fresnel_dielectric_ext/{eta:.6f}", live(lambda: ref.fresnel_dielectric_ext(c, eta)), len(c))
+        fp, tp = port.fresnel_dielectric_ext(c[i], eta)
         assert np.array_equal(fr, fp) and np.array_equal(tr, tp)
     for eta, k in (((0.2, 0.9, 1.1), (3.9, 2.4, 2.2)), ((1.65746, 0.880369, 0.521229), (9.22387, 6.26952, 4.837)), ((0, 0, 0), (1, 1, 1)), ((1.5, 1.5, 1.5), (0, 0, 0))):
-        assert np.array_equal(ref.fresnel_conductor_exact(np.abs(c), eta, k), port.fresnel_conductor_exact(np.abs(c), eta, k))
+        i, (fc,) = reference(f"fresnel_conductor_exact/{eta[0]}/{k[0]}", live(lambda: [ref.fresnel_conductor_exact(np.abs(c), eta, k)]), len(c))
+        assert np.array_equal(fc, port.fresnel_conductor_exact(np.abs(c[i]), eta, k))
     a = rng.normal(size=(200000, 3)).astype(np.float32); a /= np.linalg.norm(a, axis=1, keepdims=True); a[:3] = np.eye(3)
-    (br, cr), (bp, cp) = ref.coordinate_system(a), port.coordinate_system(a)
+    i, (br, cr) = reference("coordinate_system", live(lambda: ref.coordinate_system(a)), len(a))
+    bp, cp = port.coordinate_system(a[i])
     assert np.array_equal(br, bp) and np.array_equal(cr, cp)
     smp = rng.random((200000, 2), dtype=np.float32); smp[:4] = [[0.5, 0.5], [0, 0], [0.99999994, 0.5], [0.5, 0]]
-    assert np.array_equal(ref.square_to_cosine_hemisphere(smp), port.square_to_cosine_hemisphere(smp))
+    i, (wr,) = reference("square_to_cosine_hemisphere", live(lambda: [ref.square_to_cosine_hemisphere(smp)]), len(smp))
+    assert np.array_equal(wr, port.square_to_cosine_hemisphere(smp[i]))
 
 
-@pytest.mark.skipif(not __import__("os").path.exists(O.MFREF_SO), reason="oracle/_ref/libmicrofacet_ref.so not built (needs /root/reference at build time)")
 def test_restated_triangle_test_and_spline_equal_the_reference():
     """struct TriAccel (include/mitsuba/render/triaccel.h: Wald's precomputation `load` and `rayIntersect`) and evalCubicInterp1D (src/libcore/spline.cpp:23-60, the
     rough-transmittance lookup of roughplastic), compiled verbatim, against triaccel_load / triaccel_intersect / rough_transmittance of the oracle: the projection axis, the
     nine constants, the hit decision and (t, u, v) agree bit for bit -- the numbers every intersection of oracle and CUDA path (same operations) starts from."""
     import ctypes as C
-    ref = C.CDLL(O.MFREF_SO); port = O.load("port")
+    ref = C.CDLL(O.MFREF_SO) if HAVE_MFREF else None; port = O.load("port")
+    live = lambda f: f if HAVE_MFREF else None
     f32p = C.POINTER(C.c_float)
     rng = np.random.default_rng(21)
     n = 300000
@@ -212,42 +226,44 @@ def test_restated_triangle_test_and_spline_equal_the_reference():
     o = (tgt + rng.normal(size=(n, 3)) * 5).astype(np.float32); d = (tgt - o); d /= np.linalg.norm(d, axis=1, keepdims=True); d = d.astype(np.float32)
     d[200:300] = (B - A)[200:300] / np.linalg.norm((B - A)[200:300], axis=1, keepdims=True)
     mint = np.full(n, 1e-4, np.float32); maxt = np.where(rng.random(n) < 0.1, 3.0, np.inf).astype(np.float32)
-    outs = []
-    for lib, name in ((ref, "mfref_triaccel"), (port, "ppgo_triaccel")):
-        k = np.zeros(n, np.int32); c9 = np.zeros((n, 9), np.float32); hit = np.zeros(n, np.uint8); tuv = np.zeros((n, 3), np.float32)
+    def run(lib, name, sel):
+        args = [np.ascontiguousarray(a[sel], np.float32) for a in (A, B, Cc, o, d, mint, maxt)]; m = len(args[0])
+        k = np.zeros(m, np.int32); c9 = np.zeros((m, 9), np.float32); hit = np.zeros(m, np.uint8); tuv = np.zeros((m, 3), np.float32)
         fn = getattr(lib, name); fn.argtypes = [C.c_size_t] + [f32p] * 7 + [C.POINTER(C.c_int), f32p, C.POINTER(C.c_ubyte), f32p]
-        args = [np.ascontiguousarray(a, np.float32) for a in (A, B, Cc, o, d, mint, maxt)]
-        fn(n, *[a.ctypes.data_as(f32p) for a in args], k.ctypes.data_as(C.POINTER(C.c_int)), c9.ctypes.data_as(f32p), hit.ctypes.data_as(C.POINTER(C.c_ubyte)), tuv.ctypes.data_as(f32p))
-        outs.append((k, c9, hit, tuv))
-    (k0, c0, h0, t0), (k1, c1, h1, t1) = outs
-    assert np.array_equal(k0, k1) and (k0[100:200] == 3).all() and 0.1 < h0.mean() < 0.5
+        fn(m, *[a.ctypes.data_as(f32p) for a in args], k.ctypes.data_as(C.POINTER(C.c_int)), c9.ctypes.data_as(f32p), hit.ctypes.data_as(C.POINTER(C.c_ubyte)), tuv.ctypes.data_as(f32p))
+        return k, c9, hit, tuv
+    i, (k0, c0, h0, t0) = reference("triaccel", live(lambda: run(ref, "mfref_triaccel", slice(None))), n)
+    k1, c1, h1, t1 = run(port, "ppgo_triaccel", i)
+    assert np.array_equal(k0, k1) and (k0[(i >= 100) & (i < 200)] == 3).all() and 0.1 < h0.mean() < 0.5
     ok = k0 < 3
     assert np.array_equal(c0[ok].view(np.uint32), c1[ok].view(np.uint32))             # (bit patterns: NaN-free here, and -0.0 must stay -0.0)
     assert np.array_equal(h0, h1) and np.array_equal(t0[h0 == 1], t1[h0 == 1])
     # spline: the 100-entry transmittance table of a material, looked up at |cos|^(1/4) and clamped to [0, 1] (rtrans.h:183-193, 233)
-    if not __import__("os").path.exists("/root/reference/mitsuba/data/microfacet/ggx.dat"):
-        return                                                              # (the table comes from the reference's data files)
     from ppg_b200 import rtrans
     lut, _ = rtrans.reduce_for_material("ggx", 1.5, 0.2)
     lut = np.ascontiguousarray(lut, np.float32)
     cs = np.concatenate([rng.random(100000), [0.0, 1.0, 1e-8]]).astype(np.float32)
-    ref.mfref_cubic_interp_1d.argtypes = [C.c_size_t, f32p, f32p, C.c_size_t, C.c_float, C.c_float, f32p]
     port.ppgo_rough_transmittance.argtypes = [C.c_size_t, f32p, f32p, f32p]
     x = np.power(np.abs(cs), np.float32(0.25)).astype(np.float32)
-    a = np.zeros_like(cs); b = np.zeros_like(cs)
-    ref.mfref_cubic_interp_1d(len(cs), x.ctypes.data_as(f32p), lut.ctypes.data_as(f32p), len(lut), 0.0, 1.0, a.ctypes.data_as(f32p))
-    port.ppgo_rough_transmittance(len(cs), cs.ctypes.data_as(f32p), lut.ctypes.data_as(f32p), b.ctypes.data_as(f32p))
+    def spline():
+        a = np.zeros_like(cs)
+        ref.mfref_cubic_interp_1d.argtypes = [C.c_size_t, f32p, f32p, C.c_size_t, C.c_float, C.c_float, f32p]
+        ref.mfref_cubic_interp_1d(len(cs), x.ctypes.data_as(f32p), lut.ctypes.data_as(f32p), len(lut), 0.0, 1.0, a.ctypes.data_as(f32p))
+        return [a]
+    i, (a,) = reference("cubic_interp_1d", live(spline), len(cs))
+    csi = np.ascontiguousarray(cs[i]); b = np.zeros_like(csi)
+    port.ppgo_rough_transmittance(len(csi), csi.ctypes.data_as(f32p), lut.ctypes.data_as(f32p), b.ctypes.data_as(f32p))
     # (the abscissa |cos|^(1/4) is computed by numpy for the reference function and by libm's powf inside the restatement: equal in most cases, one ulp apart otherwise)
     assert np.abs(np.clip(a, 0, 1) - b).max() <= 2e-6 and (np.clip(a, 0, 1) == b).mean() > 0.9
 
 
-@pytest.mark.skipif(not __import__("os").path.exists(O.MFREF_SO), reason="oracle/_ref/libmicrofacet_ref.so not built (needs /root/reference at build time)")
 def test_restated_discrete_distribution_equals_the_reference():
     """struct DiscreteDistribution (include/mitsuba/core/pmf.h:35-210: append, normalize, sample, sampleReuse), compiled verbatim, against the cumulative tables the
     oracle's light sampling builds and Scene::cdfSample: the normalised entries, the sum, the chosen index and the reused sample agree bit for bit -- with zero-weight
     entries (which `sample` skips), a dominant entry and samples on the table's own boundaries."""
     import ctypes as C
-    ref = C.CDLL(O.MFREF_SO); port = O.load("port")
+    ref = C.CDLL(O.MFREF_SO) if HAVE_MFREF else None; port = O.load("port")
+    live = lambda f: f if HAVE_MFREF else None
     f32p = C.POINTER(C.c_float); u32p = C.POINTER(C.c_uint32)
     rng = np.random.default_rng(33)
     for ne in (1, 2, 7, 300):
@@ -259,12 +275,15 @@ def test_restated_discrete_distribution_equals_the_reference():
         smp = rng.random(n, dtype=np.float32)
         cdf = np.concatenate([[0], np.cumsum(w, dtype=np.float32)]); smp[:ne + 1] = np.minimum(cdf / cdf[-1], np.float32(0.99999994))     # boundaries (approximately: float32 cumsum)
         smp[ne + 1] = 0.0
-        outs = []
-        for lib, name in ((ref, "mfref_discrete"), (port, "ppgo_discrete")):
-            pdf = np.zeros(ne, np.float32); s = C.c_float(); idx = np.zeros(n, np.uint32); reuse = np.zeros(n, np.float32)
+        def run(lib, name, sel):
+            x = np.ascontiguousarray(smp[sel]); m = len(x)
+            pdf = np.zeros(ne, np.float32); s = C.c_float(); idx = np.zeros(m, np.uint32); reuse = np.zeros(m, np.float32)
             fn = getattr(lib, name); fn.argtypes = [C.c_size_t, f32p, C.c_size_t, f32p, f32p, C.POINTER(C.c_float), u32p, f32p]
-            fn(ne, w.ctypes.data_as(f32p), n, smp.ctypes.data_as(f32p), pdf.ctypes.data_as(f32p), C.byref(s), idx.ctypes.data_as(u32p), reuse.ctypes.data_as(f32p))
-            outs.append((pdf, s.value, idx, reuse))
-        (p0, s0, i0, r0), (p1, s1, i1, r1) = outs
-        assert np.array_equal(p0, p1) and s0 == s1 and np.array_equal(i0, i1) and np.array_equal(r0.view(np.uint32), r1.view(np.uint32)), ne
+            fn(ne, w.ctypes.data_as(f32p), m, x.ctypes.data_as(f32p), pdf.ctypes.data_as(f32p), C.byref(s), idx.ctypes.data_as(u32p), reuse.ctypes.data_as(f32p))
+            return pdf, np.array([s.value], np.float32), idx, reuse
+        j, (p0,) = reference(f"discrete/{ne}/pdf", live(lambda: run(ref, "mfref_discrete", slice(None))[:1]), ne)
+        _, (s0,) = reference(f"discrete/{ne}/sum", live(lambda: run(ref, "mfref_discrete", slice(None))[1:2]), 1)
+        i, (i0, r0) = reference(f"discrete/{ne}/sample", live(lambda: run(ref, "mfref_discrete", slice(None))[2:]), n)
+        p1, s1, i1, r1 = run(port, "ppgo_discrete", i)
+        assert np.array_equal(p0, p1[j]) and s0 == s1 and np.array_equal(i0, i1) and np.array_equal(r0.view(np.uint32), r1.view(np.uint32)), ne
         assert (w[i0] > 0).all()                                                   # an entry of probability 0 is never returned (pmf.h:131-134)

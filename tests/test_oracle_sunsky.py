@@ -1,30 +1,35 @@
 """The host-side bake of Mitsuba's sunsky emitter (ppg_b200/sunsky.py) against the reference's own sky model compiled verbatim
-(oracle/_ref/libskymodel_ref.so, built by `make -C oracle skyref` where /root/reference exists) and against known answers."""
+(oracle/_ref/libskymodel_ref.so, built by `make -C oracle skyref` where the original project is present; its outputs stored under tests/golden
+otherwise) and against known answers.  The Hosek-Wilkie coefficient tables come from tests/golden/sky_model_rgb.npz (tests/conftest.py)."""
 import ctypes as C
 import math
 import os
 
 import numpy as np
-import pytest
 
 from common import ROOT, load_fixture_scene
+from reference_outputs import reference
 
 SKY_REF = os.path.join(ROOT, "oracle", "_ref", "libskymodel_ref.so")
-HAVE_TABLES = os.path.exists("/root/reference/mitsuba/src/emitters/sunsky/skymodeldata.h")
 KITCHEN_PROPS = dict(hour="9", turbidity="5", sunRadiusScale="4", scale="50")      # scenes/kitchen/kitchen-improved.xml:2930-2938
 
 
-@pytest.mark.skipif(not (HAVE_TABLES and os.path.exists(SKY_REF)), reason="reference sky model not built")
 def test_sky_model_matches_the_reference_code():
     """arhosek_rgb_skymodelstate_alloc_init + arhosek_tristim_skymodel_radiance (src/emitters/sunsky/skymodel.cpp:329-381) vs the restatement."""
     from ppg_b200 import sunsky
-    lib = C.CDLL(SKY_REF); lib.skyref_rgb.restype = C.c_double; lib.skyref_rgb.argtypes = [C.c_double] * 5 + [C.c_int]
     T = sunsky._sky_tables()
     rng = np.random.default_rng(1)
+    args = []
     for k in range(300):
         turb = 10.0 if k == 0 else (float(int(rng.uniform(1, 10))) if k < 20 else rng.uniform(1, 10))
         alb, el = rng.uniform(0, 1), rng.uniform(0, math.pi / 2); th, ga, ch = rng.uniform(0, math.pi / 2 - 1e-3), rng.uniform(0, math.pi), int(rng.integers(3))
-        ref = lib.skyref_rgb(turb, alb, el, th, ga, ch)
+        args.append((turb, alb, el, th, ga, ch))
+    def live():
+        lib = C.CDLL(SKY_REF); lib.skyref_rgb.restype = C.c_double; lib.skyref_rgb.argtypes = [C.c_double] * 5 + [C.c_int]
+        return [np.array([lib.skyref_rgb(*a) for a in args])]
+    rows, (refs,) = reference("sky_model_rgb", live if os.path.exists(SKY_REF) else None, len(args))
+    for k, ref in zip(rows, refs):
+        turb, alb, el, th, ga, ch = args[k]
         cfg, rad = sunsky.cook_configuration(T[f"datasetRGB{ch + 1}"], T[f"datasetRGBRad{ch + 1}"], turb, alb, el)
         mine = float(sunsky.sky_radiance_internal(cfg, np.float64(th), np.float64(ga)) * rad)
         assert abs(mine - ref) <= 1e-12 * max(abs(ref), 1e-9), (turb, alb, el, th, ga, ch)
@@ -42,7 +47,6 @@ def test_sun_position_known_answers():
     assert abs(math.degrees(eln) - (35.6894 - 22.2)) < 0.3 and abs(math.degrees(azn) - 180) < 3
 
 
-@pytest.mark.skipif(not HAVE_TABLES, reason="reference tree not present")
 def test_kitchen_environment_map_is_the_baked_sunsky():
     """The fixture's environment map is what sunsky.bake produces for kitchen.xml's emitter; physical sanity of the bake: nothing below the
     horizon, the sun texels hold the splatted disc (sunsky.cpp:160-207) and fit half precision (envmap.cpp:102-103), and the integrated sun
@@ -73,7 +77,6 @@ def test_low_discrepancy_points_of_the_sun_splat():
     assert np.allclose(sunsky._sobol2(i), [0, 0.5, 0.75, 0.25, 0.625, 0.125, 0.375, 0.875])      # direction numbers v ^= v >> 1
 
 
-@pytest.mark.skipif(not HAVE_TABLES, reason="reference tree not present")
 def test_sky_and_sun_emitters_are_the_two_halves_of_sunsky(tmp_path):
     """The loader bakes <emitter type="sky"> (src/emitters/sky.cpp) and <emitter type="sun"> (src/emitters/sun.cpp:142-225) with the same code as sunsky, which
     nests exactly these two (sunsky.cpp:122-207): their maps add up to the sunsky map, `scale` acts like skyScale / sunScale."""
