@@ -413,6 +413,21 @@ int ppg_op_dtree_record(int device,
                         const uint32_t *rec_tree, const float *rec_dir, const float *rec_radiance,
                         const float *rec_wo_pdf, const float *rec_weight, size_t n, int filter);
 
+/* The sampling-fraction replay of a commit launch (adam_hist -> exclusive_scan -> adam_scatter -> adam_seq -> adam_progress, with the
+ * launch shapes the renderer uses) on given records, for testing it against the reference's AdamOptimizer.
+ * states: 6 floats per leaf (iter, m, v, variable, batchAcc, batchGrad), the start of the first batch.  Records as the commit kernel
+ * appends them: rec_a 4 floats {bits(leaf), product, woPdf, bsdfPdf}, rec_b 2 floats {dTreePdf, weight}; counts[b * replicas + r]
+ * records of batch b, replica r follow each other in that order.  Of a group of `total` records the first min(total, cap) are
+ * replayed, as in a commit launch with a record list of capacity cap.  The batches run one after the other on the same counting
+ * buffers.  replicas > 1 or merge != 0: every replica replays its records from the state at the start of the batch, then
+ * adam_pack, a sum over the replicas in replica order (standing in for the allreduce) and adam_merge.  loss = PPG_LOSS_KL | VAR.
+ * Outputs, per batch (any may be NULL): states_out 6 floats per leaf; replica_out 6 floats per leaf per replica before the merge;
+ * theta_out the variable written into the leaf record; sorted_a_out / sorted_b_out the bucketed record lists (layout of rec_a /
+ * rec_b, min(total, cap) entries per group); progress_out {sum steps * |f after - f before| * 2^20, sum steps}. */
+int ppg_op_fraction_replay(int device, const float *states, size_t n_leaves, const float *rec_a, const float *rec_b, const size_t *counts,
+                           int n_batches, int replicas, int merge, size_t cap, int loss, float *states_out, float *replica_out, float *theta_out,
+                           float *sorted_a_out, float *sorted_b_out, unsigned long long *progress_out);
+
 /* The acceleration structure ppg_set_scene builds over the scene's triangles (binned-SAH BVH; it takes the place of the reference's ShapeKDTree,
  * src/librender/skdtree.cpp), on the HOST alone -- no CUDA device needed: for tests of the builder and for timing it.  positions 3 floats per vertex,
  * indices 3 per triangle; threads <= 0: the library's default (the cores this process may use, at most 16; PPG_HOST_THREADS overrides).

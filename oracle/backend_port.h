@@ -78,6 +78,10 @@ struct PortBackend {
         const Adam &a = t.nodes[i].dTree.opt;
         out6[0] = (float) a.iter; out6[1] = a.m1; out6[2] = a.m2; out6[3] = a.variable; out6[4] = a.batchAcc; out6[5] = a.batchGrad;
     }
+    void setAdamState(size_t i, const float *in6) {
+        Adam &a = t.nodes[i].dTree.opt;
+        a.iter = (int) in6[0]; a.m1 = in6[1]; a.m2 = in6[2]; a.variable = in6[3]; a.batchAcc = in6[4]; a.batchGrad = in6[5];
+    }
     void aabb(float *mn, float *mx) const { mn[0] = t.amin.x; mn[1] = t.amin.y; mn[2] = t.amin.z; mx[0] = t.amax.x; mx[1] = t.amax.y; mx[2] = t.amax.z; }
 
     // flat [building sums (4 per quadtree node) | building weight] per leaf in node order (the exchange buffer of SURVEY 8e)

@@ -328,6 +328,13 @@ int ppgo_tree_fraction(ppgo_handle *h, size_t n, const uint32_t *leaf, float *fr
     for (size_t i = 0; i < n; ++i) frac_out[i] = T.bsdfSamplingFraction(T.leafAt(leaf[i]));
     return PPG_OK;
 }
+// seed the sampling-fraction optimiser of S-tree node `node` (6 floats: iter, m, v, variable, batchAcc, batchGrad)
+int ppgo_tree_set_adam(ppgo_handle *h, uint32_t node, const float state6[6]) {
+    BackendT &T = h->T();
+    if (node >= T.numNodes() || !T.isLeaf(node)) return PPG_ERR_INVALID_ARGUMENT;
+    T.setAdamState(node, state6);
+    return PPG_OK;
+}
 int ppgo_tree_counts(ppgo_handle *h, uint64_t counts[4]) {
     BackendT &T = h->T();
     counts[0] = T.numNodes(); counts[1] = counts[2] = counts[3] = 0;

@@ -79,6 +79,8 @@ int ppgo_tree_pdf(ppgo_handle *h, size_t n, const uint32_t *leaf, const float *d
 int ppgo_tree_sample(ppgo_handle *h, size_t n, const uint32_t *leaf, const float *rnd, size_t rnd_stride, float *dir_out);
 int ppgo_tree_fraction(ppgo_handle *h, size_t n, const uint32_t *leaf, float *frac_out);
 /* counts[0]=S-tree nodes, [1]=leaves, [2]=total sampling quadtree nodes, [3]=total building quadtree nodes */
+/* Seed the sampling-fraction optimiser (AdamOptimizer::State) of leaf `node`: iter, m, v, variable, batchAcc, batchGrad. */
+int ppgo_tree_set_adam(ppgo_handle *h, uint32_t node, const float state6[6]);
 int ppgo_tree_counts(ppgo_handle *h, uint64_t counts[4]);
 /* export: s_children 2*N u32 (0,0 for leaves), s_axis N i32, s_is_leaf N u8;
  * per S-tree node i (valid for leaves): tree_first[which][i], tree_count, tree_sum, tree_weight, tree_depth;

@@ -93,6 +93,10 @@ struct RefBackend {
         const auto &s = t->m_nodes[i].dTree.bsdfSamplingFractionOptimizer.m_state;
         out6[0] = (float) s.iter; out6[1] = s.firstMoment; out6[2] = s.secondMoment; out6[3] = s.variable; out6[4] = s.batchAccumulation; out6[5] = s.batchGradient;
     }
+    void setAdamState(size_t i, const float *in6) {
+        auto &s = t->m_nodes[i].dTree.bsdfSamplingFractionOptimizer.m_state;
+        s.iter = (int) in6[0]; s.firstMoment = in6[1]; s.secondMoment = in6[2]; s.variable = in6[3]; s.batchAccumulation = in6[4]; s.batchGradient = in6[5];
+    }
     void aabb(float *mn, float *mx) const { const mitsuba::AABB &a = t->aabb(); for (int i = 0; i < 3; ++i) { mn[i] = a.min[i]; mx[i] = a.max[i]; } }
     size_t packSize() const { size_t n = 0; for (const auto &nd : t->m_nodes) if (nd.isLeaf) n += 4 * nd.dTree.building.numNodes() + 1; return n; }
     void packBuilding(float *buf, bool unpack) {

@@ -1928,6 +1928,77 @@ extern "C" int ppg_op_dtree_record(int device, float *sums_inout, const uint16_t
     CK(cudaMemcpy(tree_weight_inout, dwt.b.p, 4 * n_trees, cudaMemcpyDeviceToHost));
     return PPG_OK;
 }
+__global__ void op_sum_kernel(float *acc, const float *x, size_t n) {
+    for (size_t i = blockIdx.x * (size_t) blockDim.x + threadIdx.x; i < n; i += (size_t) gridDim.x * blockDim.x) acc[i] += x[i];
+}
+// The sampling-fraction replay of render_batch on caller-given records: the same kernels, in the same order, with the same launch shapes.
+extern "C" int ppg_op_fraction_replay(int device, const float *states, size_t n_leaves, const float *rec_a, const float *rec_b, const size_t *counts,
+                                      int n_batches, int replicas, int merge, size_t cap, int loss, float *states_out, float *replica_out, float *theta_out,
+                                      float *sorted_a_out, float *sorted_b_out, unsigned long long *progress_out) {
+  return guarded("ppg_op_fraction_replay", [&]() -> int {
+    if (!states || !counts || !n_leaves || n_leaves >= 0xFFFFFFFFull || n_batches < 1 || replicas < 1 || !cap || cap >= 0xFFFFFFFFull ||
+        (loss != PPG_LOSS_KL && loss != PPG_LOSS_VAR))
+        return fail(PPG_ERR_INVALID_ARGUMENT, "ppg_op_fraction_replay: bad arguments");
+    const size_t R = (size_t) replicas, L = n_leaves;
+    const bool doMerge = replicas > 1 || merge != 0;
+    size_t nTotal = 0;
+    for (size_t g = 0; g < (size_t) n_batches * R; ++g) nTotal += counts[g];
+    if (nTotal && (!rec_a || !rec_b)) return fail(PPG_ERR_INVALID_ARGUMENT, "ppg_op_fraction_replay: null records");
+    for (size_t i = 0; i < nTotal; ++i) { uint32_t leaf; memcpy(&leaf, rec_a + 4 * i, 4); if (leaf >= L) return fail(PPG_ERR_INVALID_ARGUMENT, "ppg_op_fraction_replay: leaf index out of range"); }
+    int rc = op_device(device); if (rc) return rc;
+    int dev = 0, numSMs = 0; CK(cudaGetDevice(&dev)); CK(cudaDeviceGetAttribute(&numSMs, cudaDevAttrMultiProcessorCount, dev));
+    const uint32_t nNodes = (uint32_t) L;
+    Up<float> dAdam; Up<uint32_t> dNodes;
+    if (dAdam.up(states, 6 * L) || dNodes.up(&nNodes, 1)) return fail(PPG_ERR_CUDA, "upload failed");
+    DevBuf<float4> dLeafA, dRecA, dSortA; DevBuf<float2> dRecB, dSortB; DevBuf<uint32_t> dCount, dCursor, dOffset, dScalars;
+    DevBuf<float> dBefore, dStart, dOut6, dSum6; DevBuf<unsigned long long> dProgress;
+    CK(dLeafA.alloc(L)); CK(dCount.alloc(L)); CK(dCursor.alloc(L)); CK(dOffset.alloc(L)); CK(dScalars.alloc(2)); CK(dBefore.alloc(4 * L)); CK(dProgress.alloc(2));
+    CK(dRecA.alloc(cap)); CK(dRecB.alloc(cap)); CK(dSortA.alloc(cap)); CK(dSortB.alloc(cap));
+    if (doMerge) { CK(dStart.alloc(6 * L)); CK(dOut6.alloc(6 * L)); CK(dSum6.alloc(6 * L)); }
+    CK(cudaMemset(dLeafA.p, 0, 16 * L)); CK(cudaMemset(dCount.p, 0, 4 * L)); CK(cudaMemset(dCursor.p, 0, 4 * L));     // as ensure_tree leaves them
+    MaintParams M; memset(&M, 0, sizeof(M));
+    M.adam = dAdam.b.p; M.leafA = dLeafA.p; M.nNodes = dNodes.b.p; M.capNodes = nNodes;
+    const float ratioPower = loss == PPG_LOSS_KL ? 1.0f : 2.0f;
+    std::vector<float> la(4 * L);
+    size_t first = 0;
+    for (int b = 0; b < n_batches; ++b) {
+        adam_pack_kernel<<<numSMs, 256>>>(M, nullptr, dBefore.p, nullptr, 0);
+        if (doMerge) { CK(cudaMemcpy(dStart.p, dAdam.b.p, 24 * L, cudaMemcpyDeviceToDevice)); CK(cudaMemset(dSum6.p, 0, 24 * L)); }
+        for (size_t r = 0; r < R; ++r) {
+            const size_t total = counts[(size_t) b * R + r], kept = std::min(total, cap);
+            if (r) CK(cudaMemcpy(dAdam.b.p, dStart.p, 24 * L, cudaMemcpyDeviceToDevice));
+            // the commit launch: `total` records appended, the first `cap` of them stored
+            if (kept) { CK(cudaMemcpy(dRecA.p, rec_a + 4 * first, 16 * kept, cudaMemcpyHostToDevice)); CK(cudaMemcpy(dRecB.p, rec_b + 2 * first, 8 * kept, cudaMemcpyHostToDevice)); }
+            const uint32_t total32 = (uint32_t) std::min<size_t>(total, 0xFFFFFFFFu);
+            CK(cudaMemcpy(dScalars.p, &total32, 4, cudaMemcpyHostToDevice));
+            adam_hist_kernel<<<numSMs * 4, 256>>>(dRecA.p, dScalars.p, (uint32_t) cap, dCount.p);
+            exclusive_scan_kernel<<<1, 1024>>>(dCount.p, dOffset.p, dNodes.b.p, dScalars.p + 1);
+            adam_scatter_kernel<<<numSMs * 4, 256>>>(dRecA.p, dRecB.p, dScalars.p, (uint32_t) cap, dOffset.p, dCursor.p, dSortA.p, dSortB.p);
+            adam_seq_kernel<<<numSMs * 16, 128>>>(M, dSortA.p, dSortB.p, dOffset.p, dCount.p, dCursor.p, ratioPower);
+            CK(cudaGetLastError());
+            if (kept && sorted_a_out) CK(cudaMemcpy(sorted_a_out + 4 * first, dSortA.p, 16 * kept, cudaMemcpyDeviceToHost));
+            if (kept && sorted_b_out) CK(cudaMemcpy(sorted_b_out + 2 * first, dSortB.p, 8 * kept, cudaMemcpyDeviceToHost));
+            if (replica_out) CK(cudaMemcpy(replica_out + ((size_t) b * R + r) * 6 * L, dAdam.b.p, 24 * L, cudaMemcpyDeviceToHost));
+            if (doMerge) {
+                adam_pack_kernel<<<numSMs, 256>>>(M, dOut6.p, dBefore.p, nullptr, 1);
+                op_sum_kernel<<<numSMs, 256>>>(dSum6.p, dOut6.p, 6 * L);          // the allreduce, summing the replicas in order
+            }
+            first += total;
+        }
+        if (doMerge) adam_merge_kernel<<<numSMs, 256>>>(M, dSum6.p, dBefore.p, 1.0f / (float) R, (float) (R - 1));
+        CK(cudaMemset(dProgress.p, 0, 16));
+        adam_progress_kernel<<<numSMs, 256>>>(M, dBefore.p, dProgress.p);
+        CK(cudaGetLastError());
+        if (progress_out) CK(cudaMemcpy(progress_out + 2 * b, dProgress.p, 16, cudaMemcpyDeviceToHost));
+        if (states_out) CK(cudaMemcpy(states_out + (size_t) b * 6 * L, dAdam.b.p, 24 * L, cudaMemcpyDeviceToHost));
+        if (theta_out) {
+            CK(cudaMemcpy(la.data(), dLeafA.p, 16 * L, cudaMemcpyDeviceToHost));
+            for (size_t i = 0; i < L; ++i) theta_out[(size_t) b * L + i] = la[4 * i + 2];
+        }
+    }
+    return PPG_OK;
+  });
+}
 // The acceleration structure ppg_set_scene builds, on the host alone (no CUDA device needed): for tests of the builder and for timing it.
 extern "C" int ppg_op_bvh_build(const float *positions, const uint32_t *indices, size_t n_triangles, int threads, float *nodes_out, size_t nodes_capacity,
                                 uint32_t *order_out, size_t *n_nodes_out, int *max_depth_out, double *ms_out) {

@@ -471,11 +471,67 @@ __global__ void __launch_bounds__(256) adam_scatter_kernel(const float4 *recA, c
         }
     }
 }
-// One WARP per leaf: AdamOptimizer::append / step exactly as GP:85-109, gradient as GP:672-697.  The chain over a leaf's records is sequential
-// (theta changes every ~2 records), so its speed is the latency of one link.  The 32 lanes fetch the next 32 records with coalesced loads while the
-// chain runs; every lane then walks the chain redundantly on values handed around with shuffles (no divergence, no dependent global load in the
-// chain).  The first version (one THREAD per leaf, a dependent 24-byte fetch per record) spent ~0.3 us per record: 310 of 1000 ms on SPACESHIP
-// 640x360, where the hottest leaf of an iteration holds > 100 000 records.
+// ---- the replay chain of one leaf, factored out of adam_seq_kernel so that the same source also runs host-compiled (tests/hostdev)
+// AdamOptimizer::State (GP:116-124) plus what the chain keeps between steps.  beta^iter as running double-precision products (the reference
+// evaluates std::pow(float, int) in double, GP:98-99; a pow() per step would sit on the sequential chain); the fraction f = logistic(variable)
+// and f (1 - f) are re-evaluated after a step, not per record.
+struct FractionChain {
+    int iter; float m1, m2, variable, batchAcc, batchGrad;
+    double b1pow, b2pow;
+    float f, g, fdf;          // f, 1 - f, f (1 - f)
+};
+__device__ __forceinline__ void fraction_logistic(FractionChain &s) {
+    s.f = __fdividef(1.f, 1.f + __expf(-s.variable)); s.g = 1.f - s.f; s.fdf = s.f * s.g;      // logistic (GP:64-66), fast intrinsics
+}
+// `st`: the 6 floats of MaintParams::adam (iter, m, v, variable, batchAcc, batchGrad)
+__device__ __forceinline__ FractionChain fraction_begin(const float *st) {
+    FractionChain s;
+    s.iter = (int) st[0]; s.m1 = st[1]; s.m2 = st[2]; s.variable = st[3]; s.batchAcc = st[4]; s.batchGrad = st[5];
+    s.b1pow = pow((double) 0.9f, (double) s.iter); s.b2pow = pow((double) 0.999f, (double) s.iter);
+    fraction_logistic(s);
+    return s;
+}
+__device__ __forceinline__ void fraction_end(const FractionChain &s, float *st) {
+    st[0] = (float) s.iter; st[1] = s.m1; st[2] = s.m2; st[3] = s.variable; st[4] = s.batchAcc; st[5] = s.batchGrad;
+}
+// The chain's latency is what the replay costs (the hottest leaf of SPACESHIP 1080p holds > 10^6 records per iteration), so everything that does
+// not depend on theta is taken off it: each record is reduced to {k, b, c, w} with
+//     dL/df = -ratio / woPdf * (bsdfPdf - dTreePdf),  ratio = (product / mix)^p,  mix = f * b + (1 - f) * c,  b = bsdfPdf,  c = dTreePdf
+//   KL (p = 1):  dL/df = -k / mix,      k = product * (bsdfPdf - dTreePdf) / woPdf
+//   var (p = 2): dL/df = -k / mix^2,    k = product^2 * (bsdfPdf - dTreePdf) / woPdf
+// and the chain keeps one fast division per record and {division, rsqrt, exp} per step.  The mixture is the reference's expression (GP:680), not
+// c + f (b - c): where dTreePdf > 2^24 bsdfPdf the difference loses bsdfPdf, and at a saturated fraction (f rounds to 1 for theta >= 17) that
+// mixture is exactly 0 -- an infinite dL/df times f (1 - f) = 0 made the moments NaN and pinned theta at -20 for good.
+__device__ __forceinline__ float fraction_k(float product, float woPdf, float bsdfPdf, float dTreePdf, bool var) {
+    return (var ? product * product : product) * (bsdfPdf - dTreePdf) / woPdf;
+}
+// AdamOptimizer::step (GP:97-109)
+__device__ __forceinline__ void fraction_step(FractionChain &s) {
+    const float grad = __fdividef(s.batchGrad, s.batchAcc);
+    ++s.iter; s.b1pow *= (double) 0.9f; s.b2pow *= (double) 0.999f;
+    const float lr = 0.01f * sqrtf(1.f - (float) s.b2pow) / (1.f - (float) s.b1pow);     // depends on the step count only: off the chain
+    s.m1 = 0.9f * s.m1 + (1.f - 0.9f) * grad;
+    s.m2 = 0.999f * s.m2 + (1.f - 0.999f) * grad * grad;
+    s.variable -= __fdividef(lr * s.m1, sqrtf(s.m2) + 1e-08f);
+    s.variable = fminf(fmaxf(s.variable, -20.0f), 20.0f);
+    s.batchGrad = 0.f; s.batchAcc = 0.f;
+    fraction_logistic(s);
+}
+// one record: the gradient at the current variable (optimizeBsdfSamplingFraction, GP:672-697), AdamOptimizer::append (GP:85-95) and the
+// step once the accumulated weight exceeds batchSize = 1
+__device__ __forceinline__ void fraction_link(FractionChain &s, float k, float b, float c, float w, bool var) {
+    const float mix = s.f * b + s.g * c;
+    const float dLoss_df = -__fdividef(k, var ? mix * mix : mix);
+    const float g = fmaf(dLoss_df, s.fdf, 0.01f * s.variable);
+    s.batchGrad = fmaf(g, w, s.batchGrad); s.batchAcc += w;
+    if (s.batchAcc > 1.0f) fraction_step(s);                 // batchSize = 1, GP:89
+}
+
+// One WARP per leaf.  The chain over a leaf's records is sequential (theta changes every ~2 records), so its speed is the latency of one link.
+// The 32 lanes fetch the next 32 records with coalesced loads while the chain runs; every lane then walks the chain redundantly on values handed
+// around with shuffles (no divergence, no dependent global load in the chain).  The first version (one THREAD per leaf, a dependent 24-byte fetch
+// per record) spent ~0.3 us per record: 310 of 1000 ms on SPACESHIP 640x360, where the hottest leaf of an iteration holds > 100 000 records.
+// The optimiser is not bit-reproducible in the reference either (records arrive in thread order): approximate-division rounding is far below that.
 __global__ void __launch_bounds__(128) adam_seq_kernel(MaintParams M, const float4 *recA, const float2 *recB, const uint32_t *offset, uint32_t *count,
                                                        uint32_t *cursor, float ratioPower) {
     const uint32_t nNodes = *M.nNodes;
@@ -486,51 +542,25 @@ __global__ void __launch_bounds__(128) adam_seq_kernel(MaintParams M, const floa
         if (lane == 0) { count[leaf] = 0; cursor[leaf] = 0; }              // ready for the next commit launch
         if (n == 0) continue;
         float *st = M.adam + 6 * (size_t) leaf;
-        int iter = (int) st[0]; float m1 = st[1], m2 = st[2], variable = st[3], batchAcc = st[4], batchGrad = st[5];
+        FractionChain s = fraction_begin(st);
         const uint32_t o = offset[leaf];
-        // beta^iter as running double-precision products (the reference evaluates std::pow(float, int) in double, GP:98-99);
-        // a pow() per step would sit on the sequential chain
-        double b1pow = pow((double) 0.9f, (double) iter), b2pow = pow((double) 0.999f, (double) iter);
         float4 na = make_float4(0, 0, 0, 0); float2 nb = make_float2(0, 0);
         if (lane < n) { na = __ldg(&recA[o + lane]); nb = __ldg(&recB[o + lane]); }
-        // The chain's latency is what this kernel costs (the hottest leaf of SPACESHIP 1080p holds > 10^6 records per iteration), so everything
-        // that does not depend on theta is taken off it: each lane reduces ITS record to {k, d, c, w} with
-        //     dL/df = -ratio / woPdf * (bsdfPdf - dTreePdf),  ratio = (product / mix)^p,  mix = c + f * d,  d = bsdfPdf - dTreePdf,  c = dTreePdf
-        //   KL (p = 1):  dL/df = -k / mix,      k = product * d / woPdf
-        //   var (p = 2): dL/df = -k / mix^2,    k = product^2 * d / woPdf
-        // and the chain keeps one fast division per record and {division, rsqrt, exp} per step.  The optimiser is not bit-reproducible in the
-        // reference either (records arrive in thread order): approximate-division rounding is far below that.
         const bool var = ratioPower == 2.f;
-        float f = __fdividef(1.f, 1.f + __expf(-variable)), fdf = f * (1.f - f);      // logistic (GP:64-66); re-evaluated after a step, not per record
         for (uint32_t base = 0; base < n; base += 32u) {
             const float4 ca = na; const float2 cb = nb;
             const uint32_t nxt = base + 32u + lane;
             if (nxt < n) { na = __ldg(&recA[o + nxt]); nb = __ldg(&recB[o + nxt]); }      // in flight while this chunk's chain runs
-            const float dl = ca.w - cb.x;                                                    // bsdfPdf - dTreePdf
-            const float kl = (var ? ca.y * ca.y : ca.y) * dl / ca.z;
+            const float kl = fraction_k(ca.y, ca.z, ca.w, cb.x, var);      // this lane's record, off the chain
             const uint32_t m = min(32u, n - base);
             for (uint32_t j = 0; j < m; ++j) {
-                const float k_ = __shfl_sync(0xffffffffu, kl, j), d_ = __shfl_sync(0xffffffffu, dl, j), c_ = __shfl_sync(0xffffffffu, cb.x, j), weight = __shfl_sync(0xffffffffu, cb.y, j);
-                const float mix = fmaf(f, d_, c_);
-                const float dLoss_df = -__fdividef(k_, var ? mix * mix : mix);
-                const float g = fmaf(dLoss_df, fdf, 0.01f * variable);
-                batchGrad = fmaf(g, weight, batchGrad); batchAcc += weight;
-                if (batchAcc > 1.0f) {                      // batchSize = 1, GP:89
-                    const float grad = __fdividef(batchGrad, batchAcc);
-                    ++iter; b1pow *= (double) 0.9f; b2pow *= (double) 0.999f;
-                    const float lr = 0.01f * sqrtf(1.f - (float) b2pow) / (1.f - (float) b1pow);     // depends on the step count only: off the chain
-                    m1 = 0.9f * m1 + (1.f - 0.9f) * grad;
-                    m2 = 0.999f * m2 + (1.f - 0.999f) * grad * grad;
-                    variable -= __fdividef(lr * m1, sqrtf(m2) + 1e-08f);
-                    variable = fminf(fmaxf(variable, -20.0f), 20.0f);
-                    batchGrad = 0.f; batchAcc = 0.f;
-                    f = __fdividef(1.f, 1.f + __expf(-variable)); fdf = f * (1.f - f);
-                }
+                const float k_ = __shfl_sync(0xffffffffu, kl, j), b_ = __shfl_sync(0xffffffffu, ca.w, j), c_ = __shfl_sync(0xffffffffu, cb.x, j), w_ = __shfl_sync(0xffffffffu, cb.y, j);
+                fraction_link(s, k_, b_, c_, w_, var);
             }
         }
         if (lane == 0) {
-            st[0] = (float) iter; st[1] = m1; st[2] = m2; st[3] = variable; st[4] = batchAcc; st[5] = batchGrad;
-            float4 la = M.leafA[leaf]; la.z = variable; M.leafA[leaf] = la;
+            fraction_end(s, st);
+            float4 la = M.leafA[leaf]; la.z = s.variable; M.leafA[leaf] = la;
         }
     }
 }

@@ -220,6 +220,8 @@ def load_library(path: str | None = None):
     lib.ppg_op_dtree_pdf.argtypes = [C.c_int, f32p, u16p, C.c_size_t, u32p, f32p, f32p, C.c_size_t, u32p, f32p, C.c_size_t, f32p]
     lib.ppg_op_dtree_sample.argtypes = [C.c_int, f32p, u16p, C.c_size_t, u32p, f32p, f32p, C.c_size_t, u32p, f32p, C.c_size_t, C.c_size_t, f32p]
     lib.ppg_op_dtree_record.argtypes = [C.c_int, f32p, u16p, C.c_size_t, u32p, f32p, C.c_size_t, u32p, f32p, f32p, f32p, f32p, C.c_size_t, C.c_int]
+    lib.ppg_op_fraction_replay.argtypes = [C.c_int, f32p, C.c_size_t, f32p, f32p, C.POINTER(C.c_size_t), C.c_int, C.c_int, C.c_int, C.c_size_t, C.c_int,
+                                           f32p, f32p, f32p, f32p, f32p, C.POINTER(C.c_ulonglong)]
     lib.ppg_op_stree_lookup.argtypes = [C.c_int, u32p, C.c_size_t, f32p, f32p, f32p, C.c_size_t, u32p, f32p]
     lib.ppg_op_bvh_build.argtypes = [f32p, u32p, C.c_size_t, C.c_int, f32p, C.c_size_t, u32p, C.POINTER(C.c_size_t), C.POINTER(C.c_int), C.POINTER(C.c_double)]
     lib.ppg_op_emitter_sample_direct.argtypes = [H, C.c_size_t, f32p, f32p, f32p, C.c_int, f32p, f32p, f32p, f32p]
@@ -233,5 +235,5 @@ EXPORTED_SYMBOLS = [
     "ppg_params_default", "ppg_params_set", "ppg_params_validate", "ppg_description", "ppg_abi_version", "ppg_create",
     "ppg_destroy", "ppg_scene_file_load", "ppg_scene_file_free", "ppg_set_scene", "ppg_set_shard", "ppg_set_allreduce", "ppg_nccl_unique_id", "ppg_nccl_init", "ppg_set_clock", "ppg_set_film_callback", "ppg_render", "ppg_render_device", "ppg_cancel",
     "ppg_copy_from_device", "ppg_dump_sdtree", "ppg_set_destination", "ppg_get_moment_images", "ppg_last_error", "ppg_op_dtree_pdf", "ppg_op_dtree_sample",
-    "ppg_op_dtree_record", "ppg_op_stree_lookup", "ppg_op_emitter_sample_direct", "ppg_op_env_pdf", "ppg_op_bvh_build",
+    "ppg_op_dtree_record", "ppg_op_fraction_replay", "ppg_op_stree_lookup", "ppg_op_emitter_sample_direct", "ppg_op_env_pdf", "ppg_op_bvh_build",
 ]

@@ -229,6 +229,25 @@ def op_dtree_record(sums, children, tree_first, tree_weight, rec_tree, rec_dir, 
     return sums, tw
 
 
+def op_fraction_replay(states, rec_a, rec_b, counts, loss, cap=None, replicas=1, merge=False, device=0):
+    """The renderer's sampling-fraction replay (ppg_op_fraction_replay) on given records.  states (L, 6); rec_a (n, 4) float32 with the leaf
+    index's bits in column 0; rec_b (n, 2); counts (batches, replicas) records per group, stored in that order.  Returns a dict of per-batch
+    arrays: states (B, L, 6), replicas (B, R, L, 6), theta (B, L), sorted_a / sorted_b (the bucketed lists, rec_a / rec_b layout), progress (B, 2)."""
+    lib = capi.load_library()
+    st = np.ascontiguousarray(states, np.float32); ra = np.ascontiguousarray(rec_a, np.float32).reshape(-1, 4); rb = np.ascontiguousarray(rec_b, np.float32).reshape(-1, 2)
+    cnt = np.ascontiguousarray(np.asarray(counts, np.uint64).reshape(-1, replicas), np.uint64)
+    B, L = cnt.shape[0], len(st)
+    assert int(cnt.sum()) == len(ra) == len(rb)
+    cap = int(cap if cap is not None else max(int(cnt.max()), 1))
+    out = dict(states=np.zeros((B, L, 6), np.float32), replicas=np.zeros((B, replicas, L, 6), np.float32), theta=np.zeros((B, L), np.float32),
+               sorted_a=np.zeros_like(ra), sorted_b=np.zeros_like(rb), progress=np.zeros((B, 2), np.uint64))
+    code = {"kl": 1, "var": 2}[loss] if isinstance(loss, str) else int(loss)
+    _check(lib, lib.ppg_op_fraction_replay(device, _p(st, C.c_float), L, _p(ra, C.c_float), _p(rb, C.c_float), _p(cnt, C.c_size_t), B, replicas, int(merge), cap, code,
+                                           _p(out["states"], C.c_float), _p(out["replicas"], C.c_float), _p(out["theta"], C.c_float),
+                                           _p(out["sorted_a"], C.c_float), _p(out["sorted_b"], C.c_float), _p(out["progress"], C.c_ulonglong)))
+    return out
+
+
 def op_bvh_build(positions, indices, threads=0):
     """The BVH ppg_set_scene builds, on the host (no device): (nodes (N,8) float32, order (T,) uint32, max depth, milliseconds)."""
     lib = capi.load_library()

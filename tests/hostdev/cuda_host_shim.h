@@ -24,7 +24,7 @@ static inline double __dmul_rn(double a, double b) { return a * b; }          //
 static inline double __dadd_rn(double a, double b) { return a + b; }
 static inline double __dsub_rn(double a, double b) { return a - b; }
 #define __expf(x) expf(x)                                                      /* fast-math exp on the device (only where stated in the kernels); glibc declares but does not export the name */
-static inline float __fdividef(float a, float b) { return a / b; }            // approximate on the device; only the conservative pre-filter of the tiny-scene test uses it
+static inline float __fdividef(float a, float b) { return a / b; }            // approximate on the device (<= 2 ulp): the conservative pre-filter of the tiny-scene test and the Adam chain (fraction_link) use it
 static inline unsigned __ballot_sync(unsigned, int p) { return p ? 1u : 0u; }
 static inline unsigned __match_any_sync(unsigned, unsigned long long) { return 1u; }
 template <class T> static inline T __shfl_sync(unsigned, T v, int) { return v; }

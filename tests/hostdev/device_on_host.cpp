@@ -136,5 +136,21 @@ int dev_dtree(const float *sums, const uint16_t *children, size_t n_nodes, const
     }
     return 0;
 }
+// the sampling-fraction replay of adam_seq_kernel (fraction_begin / fraction_k / fraction_link / fraction_end), walked sequentially over records in array
+// order: each leaf replays its records in the order they appear.  states 6 floats per leaf (in/out); rec_a 4 floats {bits(leaf), product, woPdf, bsdfPdf},
+// rec_b 2 floats {dTreePdf, weight} per record, as record_into_leaf appends them
+int dev_fraction_replay(float *states, size_t n_leaves, const float *rec_a, const float *rec_b, size_t n, int loss) {
+    const bool var = loss == PPG_LOSS_VAR;
+    std::vector<FractionChain> chain(n_leaves); std::vector<char> live(n_leaves, 0);
+    for (size_t i = 0; i < n; ++i) {
+        const uint32_t leaf = __float_as_uint(rec_a[4 * i]);
+        if (leaf >= n_leaves) return 1;
+        if (!live[leaf]) { chain[leaf] = fraction_begin(states + 6 * (size_t) leaf); live[leaf] = 1; }
+        const float product = rec_a[4 * i + 1], woPdf = rec_a[4 * i + 2], bsdfPdf = rec_a[4 * i + 3], dTreePdf = rec_b[2 * i], weight = rec_b[2 * i + 1];
+        fraction_link(chain[leaf], fraction_k(product, woPdf, bsdfPdf, dTreePdf, var), bsdfPdf, dTreePdf, weight, var);
+    }
+    for (size_t l = 0; l < n_leaves; ++l) if (live[l]) fraction_end(chain[l], states + 6 * l);
+    return 0;
+}
 int dev_rough_transmittance(size_t n, const float *c, const float *values, float *out) { for (size_t i = 0; i < n; ++i) out[i] = rough_transmittance(values, c[i]); return 0; }
 }

@@ -52,6 +52,8 @@ def _declare(lib):
     lib.ppgo_tree_sample.argtypes = [H, C.c_size_t, u32p, f32p, C.c_size_t, f32p]
     lib.ppgo_tree_fraction.argtypes = [H, C.c_size_t, u32p, f32p]
     lib.ppgo_tree_counts.argtypes = [H, u64p]
+    if hasattr(lib, "ppgo_tree_set_adam"):          # (a reference oracle built before this entry point existed lacks it)
+        lib.ppgo_tree_set_adam.argtypes = [H, C.c_uint32, f32p]
     lib.ppgo_tree_export.argtypes = [H, C.c_int, u32p, i32p, u8p, u64p, u32p, f32p, f32p, i32p, f32p, u16p, f32p, f32p]
     return lib
 
@@ -266,6 +268,11 @@ class Oracle:
         out = np.zeros((len(leaf), 3), np.float32)
         self.lib.ppgo_tree_sample(self.h, len(leaf), leaf.ctypes.data_as(C.POINTER(C.c_uint32)), fptr(rnd), rnd.shape[1], fptr(out))
         return out
+
+    def set_adam(self, node, state6):
+        """Seed the sampling-fraction optimiser of leaf `node` (iter, m, v, variable, batchAcc, batchGrad)."""
+        s = np.ascontiguousarray(state6, np.float32)
+        assert s.shape == (6,) and self.lib.ppgo_tree_set_adam(self.h, int(node), fptr(s)) == 0
 
     def fraction(self, leaf):
         leaf = np.ascontiguousarray(leaf, np.uint32); out = np.zeros(len(leaf), np.float32)
